@@ -24,6 +24,11 @@ Multi-GPU (torchrun, one process per GPU):
           newest reconstructed reference plane from its owner, issued on a side stream and overlapped with the step.
   --shard rows : ONE frame per step, its CTU rows dealt to the ranks (strong scaling, BASELINE configs[4]), every owner
           broadcasting its reconstructed rows afterwards.
+
+  --dump-outputs DIR : after the timed steps, rank 0 writes what the last timed step returned to its caller as
+          DIR/<name>.npy (float64, exact for these integer results; at most 64 MB, larger outputs as a fixed seeded
+          row sample whose indices are written beside it).  The inputs are seeded, so two builds run with the same
+          arguments can be compared output for output.
 """
 import argparse
 import ctypes as C
@@ -36,6 +41,8 @@ import time
 
 import numpy as np
 
+# the benchmark may run from a read-only tree: no bytecode caches next to the sources
+sys.dont_write_bytecode = True
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -252,6 +259,40 @@ def run_reference_arm(args, rank, world):
         except Exception as e:
             line["pred_cost_error"] = repr(e)
     print(json.dumps(line), flush=True)
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def sample_rows(n, k, seed):
+    """Sorted indices of a fixed, seeded sample of k of n rows (all n rows when n <= k)."""
+    if n <= k:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(seed).choice(n, k, replace=False))
+
+
+def write_outputs(out_dir, arrays):
+    """--dump-outputs: every array as out_dir/<name>.npy in float64 (the results are integers below 2**53)."""
+    arrays = {k: np.ascontiguousarray(v, np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise ValueError("outputs to dump take %d bytes, more than %d" % (total, DUMP_LIMIT))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def analysis_outputs(an):
+    """What Analyser.analyse hands its caller: per motion-search job the cost and the vector (quarter-pel), per CU the SSE,
+    the significant-coefficient count, the chosen reference and the 35 intra costs + the best mode.  A 2160p frame has
+    millions of jobs, so jobs and CUs are sampled at fixed seeded rows (job_index, cu_index)."""
+    jobs = sample_rows(an.njobs, 1 << 18, 1)
+    cus = sample_rows(an.ncu, 1 << 16, 2)
+    mvp = an.me_packed[jobs, 1].view(np.uint32)
+    return {"job_index": jobs, "me_cost": an.me_packed[jobs, 0],
+            "mv_x": (mvp & 0xffff).astype(np.uint16).view(np.int16), "mv_y": (mvp >> 16).astype(np.uint16).view(np.int16),
+            "cu_index": cus, "cu_sse": an.cu_sse[cus], "cu_numsig": an.cu_numsig[cus], "cu_ref": an.cu_ref[cus],
+            "intra_cost": an.intra_cost[cus]}
 
 
 def plane_as_tensor(torch, ptr, nbytes, device):
@@ -547,6 +588,12 @@ def run_ours(args, rank, world, local_rank):
     t_e2e = (time.perf_counter() - t0) * 1000.0
     barrier()
     clocks = sampler.stop()
+    # the host buffers now hold the last timed step's results.  With CTU rows sharded over N > 1 GPUs rank 0 holds only its
+    # own rows (the rest of its buffers was never written), so there is no whole-frame result to dump
+    if args.dump_outputs and rank == 0 and not (rows_mode and world > 1):
+        write_outputs(args.dump_outputs, analysis_outputs(an))
+    elif args.dump_outputs and rank == 0 and not args.shard_auto:
+        print("bench.py: --dump-outputs skipped: with --shard rows no rank holds the whole frame's results", file=sys.stderr)
 
     if world > 1:
         t = torch.tensor([t_res, t_e2e], dtype=torch.float64, device=dev)
@@ -754,6 +801,13 @@ def run_lookahead_ours(args, rank, world, local_rank):
     t_e2e = (time.perf_counter() - t0) * 1000.0
     barrier()
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        # what collect_batch(full=True) returned for this rank's frame-cost estimates in the last timed step
+        res = [la.fr[b]["res"][(b - p0, p1 - b)] for (p0, p1, b) in mine]
+        write_outputs(args.dump_outputs, {"triples": np.array(mine).reshape(-1, 3), "frame_cost": [r["score"] for r in res],
+                                          "cost_est_aq": [r["costEstAq"] for r in res], "intra_mbs": [r["intraMbs"] for r in res],
+                                          "lowres_costs": np.array([r["lowresCosts"] for r in res]),
+                                          "row_satds": np.array([r["rowSatds"] for r in res])})
     costs = {t: la.fr[t[2]]["res"][(t[2] - t[0], t[1] - t[2])]["score"] for t in mine}
     csum = sum(v * (1 + (t[0] * 31 + t[1] * 17 + t[2]) % 13) for t, v in costs.items())
     if world > 1:
@@ -874,7 +928,12 @@ def main():
     ap.add_argument("--no-chroma", action="store_true", help="luma-only motion estimation (round-1 line; the presets run with the chroma-SATD term)")
     ap.add_argument("--no-pred", action="store_true", help="skip the prediction-cost leg (AMVP / merge / bidir costs) of the N=1 line")
     ap.add_argument("--no-primitives", action="store_true", help="skip the per-primitive HBM GB/s table (8- and 10-bit) of the N=1 line")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results as DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the results of the project's own path (--impl ours)")
     global CFG, CFG_NAME
     CFG_NAME = args.config
     CFG = dict(CONFIGS[args.config])

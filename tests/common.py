@@ -4,6 +4,8 @@ The reference library (oracle/_ref/libx265ref{8,10}.so) is compiled from /root/r
 oracle/Makefile.ref; it is test infrastructure and travels to the GPU box as a prebuilt .so.
 """
 import ctypes as C
+import hashlib
+import json
 import os
 import numpy as np
 
@@ -75,6 +77,149 @@ def load_oracle(depth):
         L.orc_copy_cnt.restype = C.c_uint32
         _cache[key] = L
     return _cache[key]
+
+
+class Digest(str):
+    """The first 32 bits of the SHA-256 of an array's dtype, shape and bytes: what tests/golden/ref stores for arrays too
+    large to keep whole.  The table checks compare about 20000 output blocks, so longer digests would outweigh the rest of
+    the data; a wrong block still passes with probability 2**-32 only."""
+
+    @classmethod
+    def of(cls, a):
+        a = np.ascontiguousarray(a)
+        return cls(hashlib.sha256(("%s%s" % (a.dtype.str, a.shape)).encode() + a.tobytes()).hexdigest()[:8])
+
+
+def same(a, b):
+    """Exact equality of two arrays, either of which may be given by its Digest."""
+    if isinstance(a, Digest) or isinstance(b, Digest):
+        return (a if isinstance(a, Digest) else Digest.of(a)) == (b if isinstance(b, Digest) else Digest.of(b))
+    return np.array_equal(a, b)
+
+
+class _RefStandIn:
+    """Takes the place of the reference library while stored results are replayed: its entry points accept any call and
+    compute nothing, except the lambda table, which the tests also feed to the oracle (constants.cpp:33-50)."""
+
+    def __init__(self, depth):
+        self.depth = depth
+
+    def x265ref_lambda(self, qp):
+        from frame_helpers import lambda_for
+        return lambda_for(qp, self.depth)
+
+    def __getattr__(self, name):
+        fn = lambda *args: 0           # noqa: E731
+        setattr(self, name, fn)
+        return fn
+
+
+def _steps(keys):
+    """Keys "<result index>.<suffix>" as index steps and suffixes, which compress to almost nothing."""
+    idx = [int(k[:5]) for k in keys]
+    return {"step": [b - a for a, b in zip([0] + idx, idx)], "suffix": [k[5:] for k in keys]}
+
+
+def _keys(part):
+    return ["%05d%s" % (i, sfx) for i, sfx in zip(np.cumsum(part["step"], dtype=np.int64), part["suffix"])]
+
+
+class RefResults:
+    """What the reference computed in one test, in the order the test asks for it.
+
+    The tests that pin the oracle to the reference's own code run the same seeded inputs through both and compare.  The
+    reference's side is read from tests/golden/ref/<name>.npz, so the tests need neither the reference sources nor
+    oracle/_ref; `R` is then a stand-in whose calls compute nothing, and `rec(value)` returns the stored result in place
+    of `value`.  With X265_RECORD_GOLDEN=1 and oracle/_ref built (tests/golden/make_golden.py --ref), `R` is the real
+    reference library, `rec(value)` keeps `value`, and `done()` writes the file.  Integers and tuples of integers and
+    arrays up to 64 elements are stored whole, larger arrays as their Digest (compare those with `same`)."""
+
+    LIMIT = 64
+
+    def __init__(self, name, depth):
+        self.path = os.path.join(ROOT, "tests", "golden", "ref", name + ".npz")
+        self.recording = os.environ.get("X265_RECORD_GOLDEN") == "1"
+        self.n = 0
+        if self.recording:
+            self.R = load_ref(depth)
+            assert self.R is not None, "X265_RECORD_GOLDEN=1 needs oracle/_ref (build() where the reference sources are)"
+            self.out, self.small, self.hashes, self.packed = {}, {}, {}, {}
+        else:
+            self.R = _RefStandIn(depth)
+            # integers, tuples, digests and small arrays are kept in one JSON index and one byte array: a zip member
+            # each would cost more than the values
+            with np.load(self.path) as z:
+                self.stored = {k: v for k, v in z.items() if not k.startswith("_")}
+                index = json.loads(z["_index"].tobytes())
+                data, at = z["_data"].tobytes(), 0
+            self.stored.update(zip(_keys(index["small"]), index["small"]["val"]))
+            self.stored.update(zip(_keys(index["hash"]), index["hash"]["val"]))
+            for k, dt, shape in zip(_keys(index["arr"]), index["arr"]["dtype"], index["arr"]["shape"]):
+                a = np.frombuffer(data, dt, int(np.prod(shape)), at).reshape(shape)
+                self.stored[k] = a
+                at += a.nbytes
+            self.by_result = {}
+            for k in self.stored:
+                self.by_result.setdefault(k.split(".")[0], []).append(k)
+
+    def _put(self, key, v, whole=False):
+        if isinstance(v, (int, np.integer)):
+            self.small[key + ".i"] = [int(v)]
+        elif isinstance(v, tuple):
+            self.small[key + ".t"] = [int(x) for x in v]
+        elif v.size <= self.LIMIT and v.dtype.names is None:
+            self.packed[key + ".a"] = np.array(v)          # a copy: the test may reuse the buffer
+        elif v.size <= self.LIMIT or whole:
+            self.out[key + ".a"] = np.array(v)
+        else:
+            self.hashes[key + ".h"] = Digest.of(v)
+
+    def _decode(self, k):
+        v = self.stored[k]
+        return {"i": lambda: int(v[0]), "t": lambda: tuple(int(x) for x in v), "a": lambda: v, "h": lambda: Digest(str(v))}[k[-1]]()
+
+    def __call__(self, value, whole=False):
+        """The reference's result `value`: an int, a tuple of ints, an array, or a dict of those and of lists of arrays.
+        `whole` keeps arrays whole whatever their size (results the test feeds on as inputs)."""
+        key = "%05d" % self.n
+        self.n += 1
+        if self.recording:
+            items = value.items() if isinstance(value, dict) else [(None, value)]
+            for k, v in items:
+                sub = key if k is None else "%s.d.%s" % (key, k)
+                if isinstance(v, list):
+                    for i, x in enumerate(v):
+                        self._put("%s.l%d" % (sub, i), x, whole)
+                else:
+                    self._put(sub, v, whole)
+            return value
+        return self._replay(key)
+
+    def _replay(self, key):
+        # stored keys: <key>.<kind>, <key>.l<i>.<kind>, <key>.d.<field>.<kind>, <key>.d.<field>.l<i>.<kind>
+        fields = {}
+        for k in self.by_result.get(key, []):
+            parts = k[len(key) + 1:].split(".")
+            field, rest = (parts[1], parts[2:]) if parts[0] == "d" else (None, parts)
+            fields.setdefault(field, {})[int(rest[0][1:]) if len(rest) == 2 else None] = self._decode(k)
+        if not fields:
+            raise KeyError("%s: no stored result %s (regenerate with tests/golden/make_golden.py --ref)" % (self.path, key))
+        vals = {f: items[None] if None in items else [items[i] for i in range(len(items))] for f, items in fields.items()}
+        return vals[None] if None in vals else vals
+
+    def done(self):
+        """End of the test: write the recorded results, or check that every stored one was asked for."""
+        if self.recording:
+            os.makedirs(os.path.dirname(self.path), exist_ok=True)
+            index = {"small": dict(_steps(self.small), val=list(self.small.values())),
+                     "hash": dict(_steps(self.hashes), val=list(self.hashes.values())),
+                     "arr": dict(_steps(self.packed), dtype=[a.dtype.str for a in self.packed.values()],
+                                 shape=[a.shape for a in self.packed.values()])}
+            self.out["_index"] = np.frombuffer(json.dumps(index, separators=(",", ":")).encode(), np.uint8)
+            self.out["_data"] = np.frombuffer(b"".join(a.tobytes() for a in self.packed.values()), np.uint8)
+            np.savez_compressed(self.path, **self.out)
+        else:
+            assert self.n == len(self.by_result), "%s: %d results stored, %d asked for" % (self.path, len(self.by_result), self.n)
 
 
 def ref_fn(L, name, restype, argtypes, i=0, j=0, k=0):

@@ -1,6 +1,7 @@
 """Generates tests/golden/primitives_{8,10}.npz from the REAL reference (oracle/_ref/libx265ref*.so,
 compiled from /root/reference by oracle/Makefile.ref).  Run in the build container only:
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py          (primitives_*.npz, me_chroma_*.npz)
+    python tests/golden/make_golden.py --ref    (ref/*.npz, the results the *_oracle_vs_ref tests replay)
 Each entry stores the inputs and the reference's outputs, so the checks need no reference at run time."""
 import ctypes as C
 import os
@@ -98,7 +99,22 @@ def gen_chroma(depth):
     print("wrote me_chroma_%d.npz with %d jobs" % (depth, len(rows)))
 
 
+# the tests that replay the reference's results from tests/golden/ref (common.RefResults)
+REF_TESTS = ["tests/test_oracle_vs_ref.py", "tests/test_frame_oracle_vs_ref.py", "tests/test_lookahead_oracle_vs_ref.py"]
+
+
+def gen_ref_results():
+    """Rewrites tests/golden/ref/*.npz: the tests run with the reference live and record what it computed."""
+    import subprocess
+    root = os.path.dirname(os.path.dirname(HERE))
+    env = dict(os.environ, X265_RECORD_GOLDEN="1")
+    subprocess.check_call([sys.executable, "-m", "pytest", "-q", "-p", "no:cacheprovider"] + REF_TESTS, cwd=root, env=env)
+
+
 if __name__ == "__main__":
+    if "--ref" in sys.argv:
+        gen_ref_results()
+        sys.exit(0)
     for d in (8, 10):
         if "--chroma-only" not in sys.argv:
             gen(d)

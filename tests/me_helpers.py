@@ -2,7 +2,7 @@
 (oracle/_ref, motion.cpp:739) and through the oracle restatement (oracle/oracle_me.c)."""
 import ctypes as C
 import numpy as np
-from common import P, I, IP, ptr, pixel_dtype, make_plane
+from common import P, I, IP, ptr, pixel_dtype, make_plane, same
 
 MVRANGE = 65536  # +-2*BC_MAX_MV like bitcost.h:77
 
@@ -162,7 +162,7 @@ def run_both_chroma(O, R, depth, rng, w, h, method, subme, smooth, merange, qp=3
     return (cr, int(out_r[0]), int(out_r[1])), (co, int(out_o[0]), int(out_o[1]))
 
 
-def run_both_sea(O, R, depth, rng, w, h, subme, smooth, merange, qp=30):
+def run_both_sea(O, R, depth, rng, w, h, subme, smooth, merange, qp=30, rec=lambda v: v):
     """X265_SEA (motion.cpp:1242-1395) through the real MotionEstimate with the 12 integral planes FrameFilter::computeMEIntegral
     would hand it (x265ref_build_integral: the real integral_init primitives) and through the oracle (orc_build_integral +
     method 4); also checks the two sets of planes against each other over the region the search can touch."""
@@ -184,8 +184,7 @@ def run_both_sea(O, R, depth, rng, w, h, subme, smooth, merange, qp=30):
     R.x265ref_build_integral(ptr(refb, org), stride, H // 64, arr_r)
     O.orc_build_integral(ptr(refb, org), stride, H // 64, arr_o)
     rows = slice(margin - 79, margin + H + 78)
-    for a, b in zip(ipl_r, ipl_o):
-        assert np.array_equal(a[rows], b[rows])
+    assert same(rec(np.stack([a[rows] for a in ipl_r])), np.stack([b[rows] for b in ipl_o]))
     bx = int(rng.integers(0, (W - w) // 4 + 1)) * 4; by = int(rng.integers(0, (H - h) // 4 + 1)) * 4
     offset = org + by * stride + bx
     qmvp = (int(rng.integers(-40, 41)), int(rng.integers(-40, 41)))

@@ -130,19 +130,11 @@ def test_lookahead_adaptive_quant_gpu(cu, depth, lslices):
     (oracle/_ref, slicetype.cpp:444-694) uploaded as Lowres::invQscaleFactor; intra estimate and frame costs on the device
     (costEst, costEstAq, AQ-weighted row sums, with and without cooperative slices) equal the oracle, which
     tests/test_lookahead_oracle_vs_ref.py::test_lookahead_with_adaptive_quant pins to the reference."""
-    from common import load_ref
-    from frame_helpers import gen_chroma
-    from test_lookahead_oracle_vs_ref import RefLookahead
+    from test_lookahead_oracle_vs_ref import aq_inputs, AQ_TRIPLES
     from x265_b200.lookahead import Lookahead, coop_slices
-    R = load_ref(depth)
-    if R is None:
-        pytest.skip("oracle/_ref not built")
     O = load_oracle(depth)
     W, H = 1280, 720
-    frames = [gen_luma(W, H, i, bits=depth) for i in range(3)]
-    chroma = [(gen_chroma(W, H, i, 1, bits=depth), gen_chroma(W, H, i, 2, bits=depth)) for i in range(3)]
-    ref = RefLookahead(R, frames, lslices=lslices, aq=2, chroma=chroma)
-    invq = [ref.get(i, 8) for i in range(3)]
+    frames, invq, ref_costs = aq_inputs(depth, lslices)
     assert any((q != 256).any() for q in invq)
     sl = coop_slices(H, lslices)
     orc = OracleLookahead(O, frames, depth, slices=sl if sl[0] > 1 else None, invq=invq)
@@ -155,11 +147,11 @@ def test_lookahead_adaptive_quant_gpu(cu, depth, lslices):
         assert np.array_equal(la.fr[i]["intraCost"].download(np.int32), orc.fr[i]["intraCost"])
         assert np.array_equal(la.fr[i]["rs0"].download(np.int32), orc.fr[i]["rowSatds"][(0, 0)])
         assert tuple(int(x) for x in la.fr[i]["out0"].download(np.int64)) == orc.fr[i]["costEst"][(0, 0)]
-    for (p0, p1, b) in [(0, 1, 1), (0, 2, 1), (0, 2, 2)]:
+    for (p0, p1, b), ref_cost in zip(AQ_TRIPLES, ref_costs):
         a, c = la.cost(p0, p1, b), orc.cost(p0, p1, b)
         d0, d1 = b - p0, p1 - b
         r = la.fr[b]["res"][(d0, d1)]
-        assert a == c == ref.cost(p0, p1, b), (p0, p1, b)
+        assert a == c == ref_cost, (p0, p1, b)
         assert r["costEstAq"] == orc.fr[b]["costEst"][(d0, d1)][1]
         assert np.array_equal(r["rowSatds"], orc.fr[b]["rowSatds"][(d0, d1)])
         assert np.array_equal(r["lowresCosts"], orc.fr[b]["lowresCosts"][(d0, d1)])
