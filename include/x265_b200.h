@@ -261,6 +261,14 @@ int x265cu_analyser_set_ref_chroma(x265cu_analyser*, int idx, const void* cb_hos
 int x265cu_analyser_load_chroma(x265cu_analyser*, const void* cb_host, const void* cr_host, int host_stride);
 void* x265cu_analyser_recon_plane(x265cu_analyser*, int depthIdx /* 0..3 = CU 64,32,16,8 */, int* stride);
 int x265cu_analyser_recon_to_ref(x265cu_analyser*, int depthIdx, int refIdx, int ctuRow0, int ctuRow1);
+/* Quarter-pel phase planes (X265CU_ME_PHASEPLANES, default 1; 0 = the motion search interpolates every sub-pel candidate
+ * and nothing extra is allocated): every run of the ME stage first computes, per reference, the 15 fractional luma phases
+ * (luma_hpp / luma_vpp / luma_hvpp) of every position its jobs can read, and the pre-checks and the sub-pel refinement read
+ * their candidates from them.  Results are identical either way; the planes cost 15 extra planes of device memory per
+ * reference. */
+int x265cu_analyser_phase_planes_ms(x265cu_analyser*, float* ms);     /* device ms of the last run's plane build (0: none) */
+void* x265cu_analyser_ref_plane_phase(x265cu_analyser*, int idx, int phase);   /* pixel (0,0) of phase (yFrac << 2) | xFrac */
+int x265cu_analyser_phase_region(x265cu_analyser*, int idx, int box[4]);       /* built rectangle [x0, x1) x [y0, y1) */
 
 /* ---------- lookahead frame costs (BASELINE configs[1]; slicetype.cpp:696-805, 3115-3388) ----------
  * All pointers are device pointers.  Planes are the 4 lowres hpel planes of a frame (origin pixel,

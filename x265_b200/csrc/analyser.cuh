@@ -5,6 +5,7 @@
 #include "frame.cuh"
 #include "me.cuh"
 #include "me_window.cuh"
+#include "phase_planes.cuh"
 #include <vector>
 #include <stdlib.h>
 
@@ -39,9 +40,16 @@ struct x265cu_analyser
     int windowOn; MeGroup* d_groups[3]; int32_t* d_grpJobs[3]; std::vector<int> rowGrp[3];
     CUtensorMap* d_tmaps; int32_t* d_left;
     int32_t* d_order;                     // jobs of every CTU row sorted by PU shape (geometry.h)
+    // quarter-pel phase planes (phase_planes.cuh): ppOn = 0 (X265CU_ME_PHASEPLANES=0) keeps the interpolating pre-check and
+    // sub-pel kernels and allocates nothing extra.  Otherwise every d_refs[r] holds 16 planes ppitch bytes apart (plane 0 =
+    // the reference), rebuilt by every run of the ME stage over the box of positions its jobs can read (d_ppBox).
+    int ppOn; size_t ppitch; int* d_ppBox;
+    cudaEvent_t ev_pp[2]; int pp_valid;   // plane build of the last an_run
 };
 
 static const int AN_MARGIN_X = 96, AN_MARGIN_Y = 80;       // picyuv.cpp:87-88 with maxCUSize 64
+// the 8-tap support (3 before, 4 after) of every phase-plane position a job can read stays inside the allocation
+static_assert(PP_PAD + 3 <= AN_MARGIN_X && PP_PAD + 4 <= AN_MARGIN_Y, "phase-plane region exceeds the plane margins");
 
 template <typename T> static T* an_upload(x265cu_ctx* c, const std::vector<T>& v)
 {
@@ -80,12 +88,30 @@ static int an_run(x265cu_analyser* a, int stages, int r0, int r1)
     const int cu0 = a->rowCu[r0], ncu = a->rowCu[r1] - cu0;
     const int tu0 = a->rowTu[r0], ntu = a->rowTu[r1] - tu0;
     a->ev_valid = stages;
+    a->pp_valid = 0;
     CU_CHECK(cudaEventRecord(a->ev[0], c->stream));
     if ((stages & 1) && nj > 0)
     {
         k_build_me_jobs<<<(nj + 255) / 256, 256, 0, c->stream>>>(a->d_pus + job0, nj, a->d_field, a->fw, a->fh, a->p.width, a->p.height,
                                                                  a->stride, a->p.method, a->p.subme, a->p.merange, a->d_jobs + job0);
         CU_LAUNCH_CHECK(c);
+        if (a->ppOn)
+        {
+            // phase planes of every reference over the positions this slice's jobs can read (a row slice builds its band only)
+            CU_CHECK(cudaEventRecord(a->ev_pp[0], c->stream));
+            CU_CHECK(cudaMemsetAsync(a->d_ppBox, 0x7f, sizeof(int) * 4 * 16, c->stream));       // 0x7f7f7f7f: empty box
+            k_phase_plane_box<<<(nj + 255) / 256, 256, 0, c->stream>>>(a->d_jobs + job0, nj, a->stride, a->d_ppBox);
+            CU_LAUNCH_CHECK(c);
+            int reg[4];
+            phase_plane_region(a->p.width, a->p.height, reg);
+            const dim3 grid((reg[1] - reg[0] + PP_TW - 1) / PP_TW, (reg[3] - reg[2] + PP_TH - 1) / PP_TH, a->p.numRefs);
+            const int lastX = a->stride - AN_MARGIN_X - 1, lastY = a->planeRows - AN_MARGIN_Y - 1;
+            if (depth == 8) k_luma_phase_planes<uint8_t><<<grid, 256, 0, c->stream>>>((uint8_t* const*)a->d_refTable, a->stride, a->ppitch, a->d_ppBox, reg[1], reg[3], lastX, lastY);
+            else            k_luma_phase_planes<uint16_t><<<grid, 256, 0, c->stream>>>((uint8_t* const*)a->d_refTable, a->stride, a->ppitch, a->d_ppBox, reg[1], reg[3], lastX, lastY);
+            CU_LAUNCH_CHECK(c);
+            CU_CHECK(cudaEventRecord(a->ev_pp[1], c->stream));
+            a->pp_valid = 1;
+        }
         MeChromaArgs ch;
         if (a->chromaOn)
         {
@@ -107,7 +133,7 @@ static int an_run(x265cu_analyser* a, int stages, int r0, int r1)
         }
         if (launch_me(c, depth, a->d_fenc + a->orgBytes, a->stride, (const void* const*)a->d_refTable, a->stride, 0,
                       a->d_mvcost + a->mvrange, a->d_jobs + job0, nj, a->d_me_out + (size_t)job0 * 4, c->d_counter,
-                      a->chromaOn ? &ch : NULL, a->windowOn ? &win : NULL)) return -1;
+                      a->chromaOn ? &ch : NULL, a->windowOn ? &win : NULL, a->ppOn ? (int)a->ppitch : 0)) return -1;
         CU_CHECK(cudaEventRecord(a->ev[4], c->stream));      // ME search kernel alone ends here
         k_pack_me<<<(nj + 255) / 256, 256, 0, c->stream>>>(a->d_me_out + (size_t)job0 * 4, nj, a->d_me_packed + job0);
         CU_LAUNCH_CHECK(c);
@@ -169,8 +195,23 @@ x265cu_analyser* x265cu_analyser_create(x265cu_ctx* ctx, const x265cu_analysis_p
     an_build_geometry(a);
     a->d_fenc = (uint8_t*)x265cu_malloc(ctx, a->planeBytes);
     if (a->d_fenc) cudaMemset(a->d_fenc, 0, a->planeBytes);
+    // quarter-pel phase planes: 16 planes per reference allocation.  The ME kernels address a candidate by an int byte offset
+    // from its PU's origin in plane 0, which must reach the last plane's last row.
+    {
+        const char* e = getenv("X265CU_ME_PHASEPLANES");
+        a->ppOn = !(e && e[0] == '0');
+        a->ppitch = (a->planeBytes + 255) / 256 * 256;
+        if (a->ppOn && 16 * a->ppitch > (size_t)INT_MAX)
+        {
+            x265cu_set_error("analyser: phase planes do not fit int byte offsets (set X265CU_ME_PHASEPLANES=0)", cudaErrorInvalidValue, __FILE__, __LINE__);
+            delete a;
+            return NULL;
+        }
+    }
+    const size_t refBytes = a->ppOn ? 16 * a->ppitch : a->planeBytes;
     void* reft[16]; void* rect[4];
-    for (int r = 0; r < p->numRefs; r++) { a->d_refs[r] = (uint8_t*)x265cu_malloc(ctx, a->planeBytes); if (a->d_refs[r]) cudaMemset(a->d_refs[r], 0, a->planeBytes); reft[r] = a->d_refs[r] + a->orgBytes; }
+    for (int r = 0; r < p->numRefs; r++) { a->d_refs[r] = (uint8_t*)x265cu_malloc(ctx, refBytes); if (a->d_refs[r]) cudaMemset(a->d_refs[r], 0, refBytes); reft[r] = a->d_refs[r] + a->orgBytes; }
+    a->d_ppBox = a->ppOn ? (int*)x265cu_malloc(ctx, sizeof(int) * 4 * 16) : NULL;
     for (int d = 0; d < 4; d++) { a->d_recon[d] = (uint8_t*)x265cu_malloc(ctx, a->planeBytes); rect[d] = a->d_recon[d] + a->orgBytes; cudaMemset(a->d_recon[d], 0, a->planeBytes); }
     a->d_refTable = (void**)x265cu_malloc(ctx, sizeof(void*) * 16);
     a->d_reconTable = (void**)x265cu_malloc(ctx, sizeof(void*) * 4);
@@ -213,13 +254,14 @@ x265cu_analyser* x265cu_analyser_create(x265cu_ctx* ctx, const x265cu_analysis_p
     a->d_cu_ref = (int32_t*)x265cu_malloc(ctx, sizeof(int32_t) * a->ncu);
     a->d_intra = (uint32_t*)x265cu_malloc(ctx, sizeof(uint32_t) * 36 * a->ncu);
     for (int i = 0; i < 5; i++) cudaEventCreate(&a->ev[i]);
-    a->ev_valid = 0;
+    for (int i = 0; i < 2; i++) cudaEventCreate(&a->ev_pp[i]);
+    a->ev_valid = 0; a->pp_valid = 0;
     a->chromaOn = 0; a->d_refCbTable = a->d_refCrTable = NULL;
     a->d_fencC[0] = a->d_fencC[1] = NULL;
     for (int r = 0; r < 16; r++) a->d_refC[r][0] = a->d_refC[r][1] = NULL;
     a->h_fenc = (uint8_t*)x265cu_host_alloc((size_t)p->width * p->height * es);
     a->h_field = (int16_t*)x265cu_host_alloc(fieldBytes);
-    if (!a->d_intra || !a->d_coef || !a->d_me_out || !a->h_fenc || !a->h_field) return NULL;
+    if (!a->d_intra || !a->d_coef || !a->d_me_out || !a->h_fenc || !a->h_field || (a->ppOn && !a->d_ppBox)) return NULL;
     cudaDeviceSynchronize();
     return a;
 }
@@ -232,13 +274,16 @@ void x265cu_analyser_destroy(x265cu_analyser* a)
     cudaStreamSynchronize(c->stream);
     void* bufs[] = { a->d_fenc, a->d_refTable, a->d_reconTable, a->d_field, a->d_mvcost, a->d_pus, a->d_cus, a->d_tus, a->d_cu_jobs, a->d_jobs,
                      a->d_me_out, a->d_me_packed, a->d_coef, a->d_cu_sse, a->d_cu_numsig, a->d_cu_ref, a->d_intra,
-                     a->d_groups[0], a->d_groups[1], a->d_groups[2], a->d_grpJobs[0], a->d_grpJobs[1], a->d_grpJobs[2], a->d_tmaps, a->d_left, a->d_order };
+                     a->d_groups[0], a->d_groups[1], a->d_groups[2], a->d_grpJobs[0], a->d_grpJobs[1], a->d_grpJobs[2], a->d_tmaps, a->d_left, a->d_order,
+                     a->d_ppBox };
     for (void* b : bufs) cudaFree(b);
     for (int r = 0; r < a->p.numRefs; r++) cudaFree(a->d_refs[r]);
     for (int d = 0; d < 4; d++) cudaFree(a->d_recon[d]);
     for (int k = 0; k < 2; k++) { cudaFree(a->d_fencC[k]); for (int r = 0; r < a->p.numRefs; r++) cudaFree(a->d_refC[r][k]); }
     cudaFree(a->d_refCbTable); cudaFree(a->d_refCrTable);
     x265cu_host_free(a->h_fenc); x265cu_host_free(a->h_field);
+    for (int i = 0; i < 5; i++) cudaEventDestroy(a->ev[i]);
+    for (int i = 0; i < 2; i++) cudaEventDestroy(a->ev_pp[i]);
     delete a;
 }
 
@@ -379,6 +424,41 @@ int x265cu_analyser_stage_ms(x265cu_analyser* a, float* ms)
     for (int i = 0; i < 3; i++) CU_CHECK(cudaEventElapsedTime(&ms[i], a->ev[i], a->ev[i + 1]));
     ms[3] = 0.f;
     if (a->ev_valid & 1) CU_CHECK(cudaEventElapsedTime(&ms[3], a->ev[0], a->ev[4]));
+    return 0;
+}
+
+// device time (ms) of the phase-plane build of the last run (0 when it built none: planes off, or no ME stage).
+// Synchronises on it.  It lies inside stage_ms()[0].
+int x265cu_analyser_phase_planes_ms(x265cu_analyser* a, float* ms)
+{
+    *ms = 0.f;
+    if (!a->pp_valid) return 0;
+    CU_CHECK(cudaEventSynchronize(a->ev_pp[1]));
+    CU_CHECK(cudaEventElapsedTime(ms, a->ev_pp[0], a->ev_pp[1]));
+    return 0;
+}
+
+// device address of pixel (0, 0) of reference idx's quarter-pel phase plane `phase` = (yFrac << 2) | xFrac (0 = the
+// reference itself; same stride as x265cu_analyser_ref_plane).  NULL for phase > 0 when the planes are off.
+void* x265cu_analyser_ref_plane_phase(x265cu_analyser* a, int idx, int phase)
+{
+    if (idx < 0 || idx >= a->p.numRefs || phase < 0 || phase > 15 || (phase && !a->ppOn)) return NULL;
+    return a->d_refs[idx] + (size_t)phase * a->ppitch + a->orgBytes;
+}
+
+// the rectangle [box[0], box[1]) x [box[2], box[3]) (picture pixels) of reference idx's phase planes that the last run
+// built: the union of its jobs' read boxes (phase_planes.h) clipped to phase_plane_region(); empty (x0 >= x1) when
+// none.  Synchronises the stream.
+int x265cu_analyser_phase_region(x265cu_analyser* a, int idx, int* box)
+{
+    if (idx < 0 || idx >= a->p.numRefs || !a->ppOn) return -1;
+    int b[4], reg[4];
+    cudaSetDevice(a->ctx->device);
+    CU_CHECK(cudaMemcpyAsync(b, a->d_ppBox + 4 * idx, sizeof(b), cudaMemcpyDeviceToHost, a->ctx->stream));
+    CU_CHECK(cudaStreamSynchronize(a->ctx->stream));
+    phase_plane_region(a->p.width, a->p.height, reg);
+    box[0] = b[0] > reg[0] ? b[0] : reg[0]; box[1] = -b[1] < reg[1] ? -b[1] : reg[1];
+    box[2] = b[2] > reg[2] ? b[2] : reg[2]; box[3] = -b[3] < reg[3] ? -b[3] : reg[3];
     return 0;
 }
 

@@ -36,8 +36,23 @@ struct MeCtx
     bool pow2;                             // w and h are powers of two (all 2Nx2N / rect PUs); AMP sizes take the generic paths
     int nw, lgnw, lgwpr;                   // words per PU, log2, log2(words per row)
     int lgsegw;                            // log2 words per lane segment (16 B when the fenc rows allow vector loads)
+    int ppitch;                            // byte distance between quarter-pel phase planes (0: none, candidates interpolate)
     MeShared* sm;
 };
+
+// Quarter-pel phase planes (analyser.cuh, k_luma_phase_planes): the reference allocation holds 16 planes ppitch bytes
+// apart; plane (yFrac << 2) | xFrac is the reference predicted at that phase (luma_hpp / luma_vpp / luma_hvpp), so a
+// sub-pel candidate (qx, qy) is a full-pel block of plane ((qy & 3) << 2) | (qx & 3) at (qx >> 2, qy >> 2).
+template <typename P>
+__device__ __forceinline__ int me_qpel_off(const MeCtx<P>& c, int qx, int qy)       // byte offset from c.ref[0]
+{
+    return ((((qy & 3) << 2) | (qx & 3)) * c.ppitch) + ((qy >> 2) * c.rstride + (qx >> 2)) * (int)sizeof(P);
+}
+template <typename P>
+__device__ __forceinline__ const P* me_qpel_ptr(const MeCtx<P>& c, int qx, int qy)
+{
+    return (const P*)((const uint8_t*)c.ref[0] + me_qpel_off(c, qx, qy));
+}
 
 template <typename P>
 __device__ __forceinline__ int me_mvcost(const MeCtx<P>& c, int qx, int qy)
@@ -189,13 +204,10 @@ __device__ __noinline__ int me_sad_direct(const MeCtx<P>& c, const P* __restrict
     return warp_sum(acc);
 }
 
-// Full-pel SAD + mvcost of up to 32 candidate positions at once.  Lane i (< n) owns candidate i:
-// (px, py) in full-pel units relative to the block; returns that candidate's cost in lane i.
-// x8: the raster quirk (motion.cpp:1194: mvcost(tmv << 3) for every 4th column).
+// SAD of up to 32 blocks at once: lane i (< n) owns the block at byte offset offB from c.ref[0]; result in lane i
 template <typename P>
-__device__ __forceinline__ int me_eval_points(const MeCtx<P>& c, int n, int px, int py, bool x8)
+__device__ __forceinline__ int me_sad_points(const MeCtx<P>& c, int n, int offB)
 {
-    const int offB = (py * c.rstride + px) * (int)sizeof(P);          // byte offset of my candidate
     const uint8_t* rbase = (const uint8_t*)c.ref[0];
     int mysad = 0;
     if (c.pow2) mysad = me_sad_multi(c, rbase, n, offB);
@@ -208,6 +220,16 @@ __device__ __forceinline__ int me_eval_points(const MeCtx<P>& c, int n, int px, 
             if (c.lane == p) mysad = v;
         }
     }
+    return mysad;
+}
+
+// Full-pel SAD + mvcost of up to 32 candidate positions at once.  Lane i (< n) owns candidate i:
+// (px, py) in full-pel units relative to the block; returns that candidate's cost in lane i.
+// x8: the raster quirk (motion.cpp:1194: mvcost(tmv << 3) for every 4th column).
+template <typename P>
+__device__ __forceinline__ int me_eval_points(const MeCtx<P>& c, int n, int px, int py, bool x8)
+{
+    const int mysad = me_sad_points(c, n, (py * c.rstride + px) * (int)sizeof(P));
     int cost = 0x7fffffff;
     if (c.lane < n) cost = mysad + (x8 ? me_mvcost(c, px * 8, py * 8) : me_mvcost(c, px * 4, py * 4));
     return cost;
@@ -378,6 +400,10 @@ __device__ __forceinline__ void me_load_fenc(const MeCtx<P>& c, const P* __restr
     }
 }
 
+// N consecutive pixels at any alignment as ints (forward declaration: defined with the chroma helpers below)
+template <typename P, int N>
+__device__ __forceinline__ void me_ld_px(const P* __restrict__ p, int (&v)[N]);
+
 // Up to 4 sub-pel candidates of a SMALL PU, lane i (< n <= 4) owns candidate i (qx, qy) and gets its distortion.
 // Per candidate the arithmetic is exactly subpelCompare's (motion.cpp:1571-1598: luma_hpp / luma_vpp / luma_hvpp
 // = hps(rowExt) + vsp, ipfilter.cpp:79-369) followed by sad or satd (8x4 tiles, 4x4 for w = 4; pixel.cpp:263-297).
@@ -386,7 +412,8 @@ __device__ __forceinline__ void me_load_fenc(const MeCtx<P>& c, const P* __restr
 // filtered rows to shared memory (one row segment per lane-task), then every lane produces ITS row of the
 // prediction in registers, differences it against the source row, does the horizontal half of the 4x4 Hadamards
 // in registers and the vertical half with two xor-shuffle butterflies over the 4 lanes of a tile.
-template <typename P, int NPX>
+// PL: the candidates are read from the quarter-pel phase planes (no filtering, no shared memory).
+template <typename P, int NPX, bool PL>
 __device__ __forceinline__ int me_subpel_small_t(const MeCtx<P>& c, int n, int qx, int qy, bool satd)
 {
     constexpr int DEPTH = PixTraits<P>::depth;
@@ -404,7 +431,7 @@ __device__ __forceinline__ int me_subpel_small_t(const MeCtx<P>& c, int n, int q
         const int live_n = min(cpp, n - base);
         __syncwarp();
         // ---- stage 1: horizontally filtered rows of the hv candidates ----
-        for (int t0 = 0; t0 < live_n * tasksPer; t0 += 32)
+        for (int t0 = 0; !PL && t0 < live_n * tasksPer; t0 += 32)
         {
             const int t = t0 + lane;
             const int tci = min((int)(t >= tasksPer) + (int)(t >= 2 * tasksPer) + (int)(t >= 3 * tasksPer), live_n - 1);
@@ -439,7 +466,8 @@ __device__ __forceinline__ int me_subpel_small_t(const MeCtx<P>& c, int n, int q
         {
             const P* r = c.ref[0] + (mqx >> 2) + (ptrdiff_t)((mqy >> 2) + row) * c.rstride + seg * 8;
             int pr[NPX];
-            if (!(xf | yf))
+            if (PL) me_ld_px<P, NPX>(me_qpel_ptr(c, mqx, mqy) + (ptrdiff_t)row * c.rstride + seg * 8, pr);
+            else if (!(xf | yf))
             {
 #pragma unroll
                 for (int x = 0; x < NPX; x++) pr[x] = (int)__ldg(r + x);
@@ -520,14 +548,15 @@ __device__ __forceinline__ void me_load_row8(const P* __restrict__ p, int (&v)[8
 // re-use their source rows (11 rows feed 4 output rows: me_vcol4 / me_vmid4).  The PU is processed in bands of
 // BR = min(h, 1024 / w) rows (a full warp of units for w = 64 / 32 / 16 with h >= 16 / 32 / 64); hv candidates first
 // write the band's BR + 7 horizontally filtered rows to shared memory (one row segment per lane-task).
-template <typename P>
+// PL: the candidate is a full-pel block of its quarter-pel phase plane (every candidate takes the unit path of xf = yf = 0).
+template <typename P, bool PL>
 __device__ __forceinline__ int me_subpel_big(const MeCtx<P>& c, int qx, int qy, bool satd)
 {
     constexpr int DEPTH = PixTraits<P>::depth;
     const int lane = c.lane;
     const int lgsegs = c.lgw - 3, segs = 1 << lgsegs;
-    const int xf = qx & 3, yf = qy & 3;
-    const P* r0 = c.ref[0] + (qx >> 2) + (ptrdiff_t)(qy >> 2) * c.rstride;
+    const int xf = PL ? 0 : qx & 3, yf = PL ? 0 : qy & 3;
+    const P* r0 = PL ? me_qpel_ptr(c, qx, qy) : c.ref[0] + (qx >> 2) + (ptrdiff_t)(qy >> 2) * c.rstride;
     if (!(xf | yf) && !satd) return me_sad_direct(c, r0);             // full-pel SAD: the word-wise SAD core
     int16_t* mid = c.sm->mid;
     const int BR = min(c.h, 1024 >> c.lgw);
@@ -622,10 +651,10 @@ __device__ __forceinline__ int me_subpel_big(const MeCtx<P>& c, int qx, int qy, 
     return warp_sum(acc);
 }
 
-template <typename P>
+template <typename P, bool PL = false>
 __device__ __forceinline__ int me_subpel_multi_small(const MeCtx<P>& c, int n, int qx, int qy, bool satd)
 {
-    return c.w >= 8 ? me_subpel_small_t<P, 8>(c, n, qx, qy, satd) : me_subpel_small_t<P, 4>(c, n, qx, qy, satd);
+    return c.w >= 8 ? me_subpel_small_t<P, 8, PL>(c, n, qx, qy, satd) : me_subpel_small_t<P, 4, PL>(c, n, qx, qy, satd);
 }
 
 // out-of-line copy for the cold multi-site users (pre-checks, lowres band cost)
@@ -633,14 +662,22 @@ template <typename P>
 __device__ __noinline__ int me_subpel_compare(const MeCtx<P>& c, int qx, int qy, bool satd) { return me_subpel_compare_t(c, qx, qy, satd); }
 template <typename P>
 __device__ __noinline__ int me_band_cost_ni(const MeCtx<P>& c, int y0, int rows, bool satd) { return me_band_cost(c, y0, rows, satd); }
+// subpelCompare of ONE candidate out of the phase planes (AMP sizes): the full-pel compare of its phase plane
+template <typename P>
+__device__ __noinline__ int me_subpel_compare_pl(const MeCtx<P>& c, int qx, int qy, bool satd)
+{
+    const P* r = me_qpel_ptr(c, qx, qy);
+    if (!satd) return me_sad_direct(c, r);
+    return warp_satd(c.fenc, c.fstride, r, c.rstride, c.w, c.h, c.lane);
+}
 
 // PU classes of the sub-pel stage: 0 = small (pow2, w and h <= 16: four candidates at a time through
 // me_subpel_multi_small), 1 = everything else (one candidate at a time, banded).  CLS = -1 compiles both.
 template <typename P>
 __device__ __forceinline__ int me_subpel_class(const MeCtx<P>& c) { return (c.pow2 && c.w <= 16 && c.h <= 16) ? 0 : 1; }
 
-// distortion of up to 8 sub-pel candidates, lane i (< n) owns candidate i; result in lane i
-template <typename P, int CLS>
+// distortion of up to 8 sub-pel candidates, lane i (< n) owns candidate i; result in lane i.  PL: read from the phase planes.
+template <typename P, int CLS, bool PL = false>
 __device__ __forceinline__ int me_subpel_batch(const MeCtx<P>& c, int n, int qx, int qy, bool satd)
 {
     int out = 0;
@@ -650,7 +687,7 @@ __device__ __forceinline__ int me_subpel_batch(const MeCtx<P>& c, int n, int qx,
         {
             const int src = min(base + (c.lane & 3), n - 1);
             const int bqx = __shfl_sync(0xffffffffu, qx, src), bqy = __shfl_sync(0xffffffffu, qy, src);
-            int v = me_subpel_multi_small(c, min(4, n - base), bqx, bqy, satd);
+            int v = me_subpel_multi_small<P, PL>(c, min(4, n - base), bqx, bqy, satd);
             v = __shfl_sync(0xffffffffu, v, (c.lane - base) & 3);
             if (c.lane >= base && c.lane < base + 4) out = v;
         }
@@ -660,7 +697,8 @@ __device__ __forceinline__ int me_subpel_batch(const MeCtx<P>& c, int n, int qx,
         for (int k = 0; k < n; k++)
         {
             const int kqx = __shfl_sync(0xffffffffu, qx, k), kqy = __shfl_sync(0xffffffffu, qy, k);
-            int v = c.pow2 ? me_subpel_big(c, kqx, kqy, satd) : me_subpel_compare(c, kqx, kqy, satd);      // AMP sizes: generic, out of line
+            int v = c.pow2 ? me_subpel_big<P, PL>(c, kqx, kqy, satd)
+                           : PL ? me_subpel_compare_pl(c, kqx, kqy, satd) : me_subpel_compare(c, kqx, kqy, satd);      // AMP sizes: generic, out of line
             if (c.lane == k) out = v;
         }
     }
@@ -1279,8 +1317,9 @@ struct MeState { int bmx, bmy, bcost, bprecost, bestprex, bestprey; };
 #define ME_YOK(y) (((y) >= c.miny) & ((y) <= c.maxy))
 #define ME_INRANGE(x, y) ((x) >= c.minx && (x) <= c.maxx && (y) >= c.miny && (y) <= c.maxy)
 
-// phase 1 (motion.cpp:771-814): cost at the clipped MVP, at its full-pel rounding, at MV 0 and at the qpel candidates
-template <typename P, int CLS, bool CHROMA = false>
+// phase 1 (motion.cpp:771-814): cost at the clipped MVP, at its full-pel rounding, at MV 0 and at the qpel candidates.
+// PL: the luma SADs are one burst of full-pel SADs over the quarter-pel phase planes.
+template <typename P, int CLS, bool CHROMA = false, bool PL = false>
 __device__ __forceinline__ void me_phase1(MeCtx<P>& c, const x265cu_me_job& j, MeState& st, const MeChromaCtx<P>* cc = nullptr)
 {
 
@@ -1341,7 +1380,7 @@ __device__ __forceinline__ void me_phase1(MeCtx<P>& c, const x265cu_me_job& j, M
         const int cnt = 3 + j.numCand;
         valid = valid && lane < cnt;
         const int n = me_compact(valid, cnt, qx, qy, tag, dummy);
-        int cost = me_subpel_batch<P, CLS>(c, n, qx, qy, false);
+        int cost = PL ? me_sad_points(c, n, me_qpel_off(c, qx, qy)) : me_subpel_batch<P, CLS>(c, n, qx, qy, false);
         if (CHROMA && cc->on)
         {
             // the clipped MVP and the candidates go through subpelCompare (chroma term included); the MVP's full-pel
@@ -1545,8 +1584,8 @@ __device__ __forceinline__ void me_phase2(MeCtx<P>& c, const x265cu_me_job& j, M
     st.bmx = bmx; st.bmy = bmy; st.bcost = bcost;
 }
 
-// phase 3 (motion.cpp:1440-1569): pick pre-check vs search winner, sub-pel refinement
-template <typename P, int CLS, bool CHROMA = false>
+// phase 3 (motion.cpp:1440-1569): pick pre-check vs search winner, sub-pel refinement (PL: out of the phase planes)
+template <typename P, int CLS, bool CHROMA = false, bool PL = false>
 __device__ __forceinline__ void me_phase3(MeCtx<P>& c, const x265cu_me_job& j, const MeState& st, int32_t* __restrict__ out, const MeChromaCtx<P>* cc = nullptr)
 {
     const int qminy = c.miny * 4, qmaxy = c.maxy * 4;
@@ -1602,7 +1641,7 @@ __device__ __forceinline__ void me_phase3(MeCtx<P>& c, const x265cu_me_job& j, c
             int qx = bx + c_square1[i1][0] * step, qy = by + c_square1[i1][1] * step, dir = i1, dummy = 0;
             const bool valid = c.lane < dirs && (centre || !((qy < qminy) | (qy > qmaxy)));
             const int n = me_compact(valid, dirs, qx, qy, dir, dummy);
-            int cost = me_subpel_batch<P, CLS>(c, n, qx, qy, satd);
+            int cost = me_subpel_batch<P, CLS, PL>(c, n, qx, qy, satd);
             if (CHROMA && cc->on)
             {
                 const int ccost = me_chroma_batch<P, CLS>(c, *cc, n, qx, qy, n >= 32 ? 0xffffffffu : ((1u << n) - 1u));
@@ -1645,7 +1684,7 @@ __device__ __forceinline__ void me_make_ctx(MeCtx<P>& c, const x265cu_me_job& j,
     c.rstride = rstride; c.mvc = mvcost;
     c.mvpx = j.qmvp[0]; c.mvpy = j.qmvp[1];
     c.minx = j.mvmin[0]; c.miny = j.mvmin[1]; c.maxx = j.mvmax[0]; c.maxy = j.mvmax[1];
-    c.w = j.pw; c.h = j.ph; c.lgw = 31 - __clz(c.w); c.lane = lane; c.lowres = lowres; c.sm = sm;
+    c.w = j.pw; c.h = j.ph; c.lgw = 31 - __clz(c.w); c.lane = lane; c.lowres = lowres; c.sm = sm; c.ppitch = 0;
     c.pow2 = ((c.w & (c.w - 1)) | (c.h & (c.h - 1))) == 0;
     const int wpr = (c.w * (int)sizeof(P)) >> 2;            // words per row (>= 1: w >= 4)
     c.lgwpr = 31 - __clz(wpr);
@@ -1661,7 +1700,8 @@ __device__ __forceinline__ void me_make_ctx(MeCtx<P>& c, const x265cu_me_job& j,
 // because the fused body (12.4 K SASS instructions, ~200 KB) thrashes the instruction cache: ncu
 // showed 80 % of the stall samples in `no_instructions` at a 46 % i-cache hit rate, and the un-split sub-pel
 // kernel (8.8 K instructions, both PU classes resident on every SM) still sat at 64 %.  PHASE 0 = all fused
-// (the lookahead kernel's per-CU call).
+// (the lookahead kernel's per-CU call).  PL (pre-check and sub-pel launches of the frame analyser): candidates are read
+// from the quarter-pel phase planes `ppitch` bytes apart in every reference allocation; no shared-memory scratch.
 #ifndef ME_MIN_BLOCKS
 #define ME_MIN_BLOCKS 3
 #endif
@@ -1671,12 +1711,12 @@ __device__ __forceinline__ void me_make_ctx(MeCtx<P>& c, const x265cu_me_job& j,
 #ifndef ME_BIG_BLOCKS
 #define ME_BIG_BLOCKS 2          // large-PU pre-check / sub-pel kernels: 128 registers beat a third resident CTA (no spills in the tap loops)
 #endif
-template <typename P, int PHASE, int CLS>
+template <typename P, int PHASE, int CLS, bool PL = false>
 __global__ void __launch_bounds__(256, PHASE == 2 ? ME_P2_BLOCKS : (CLS == 1 ? ME_BIG_BLOCKS : ME_MIN_BLOCKS)) k_me(const P* __restrict__ fenc, int fstride, const P* const* __restrict__ refs, int rstride, int lowres,
                                                            const uint16_t* __restrict__ mvcost, const x265cu_me_job* __restrict__ jobs, int n,
                                                            int32_t* __restrict__ out, MeState* __restrict__ state, int* __restrict__ counter,
                                                            const int32_t* __restrict__ list = nullptr, const int* __restrict__ list_n = nullptr,
-                                                           const int32_t* __restrict__ order = nullptr, int order0 = 0)
+                                                           const int32_t* __restrict__ order = nullptr, int order0 = 0, int ppitch = 0)
 {
     extern __shared__ unsigned char me_smem[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -1696,15 +1736,16 @@ __global__ void __launch_bounds__(256, PHASE == 2 ? ME_P2_BLOCKS : (CLS == 1 ? M
         const x265cu_me_job j = jobs[jid];
         MeCtx<P> c;
         me_make_ctx<P>(c, j, fenc, fstride, refs, rstride, lowres, mvcost, lane, sm);
+        if (PL) c.ppitch = ppitch;
         if (CLS >= 0 && me_subpel_class(c) != CLS) continue;                   // the sibling launch owns this job
         if (PHASE == 0) me_run_job<P>(c, j, out + (size_t)jid * 4);
         else
         {
             MeState st;
             if (PHASE != 1) st = state[jid];
-            if (PHASE == 1) { me_phase1<P, CLS>(c, j, st); if (lane == 0) state[jid] = st; }
+            if (PHASE == 1) { me_phase1<P, CLS, false, PL>(c, j, st); if (lane == 0) state[jid] = st; }
             if (PHASE == 2) { me_phase2<P>(c, j, st); if (lane == 0) state[jid] = st; }
-            if (PHASE == 3) me_phase3<P, CLS>(c, j, st, out + (size_t)jid * 4);
+            if (PHASE == 3) me_phase3<P, CLS, false, PL>(c, j, st, out + (size_t)jid * 4);
         }
         __syncwarp();
     }
@@ -1712,11 +1753,11 @@ __global__ void __launch_bounds__(256, PHASE == 2 ? ME_P2_BLOCKS : (CLS == 1 ? M
 
 // The pre-check and sub-pel launches with the chroma-SATD term (x265cu_me_batch_chroma): separate instantiations, so
 // the luma-only kernels above are unchanged by it.  The integer search (phase 2) is luma only in the reference too.
-template <typename P, int PHASE, int CLS>
+template <typename P, int PHASE, int CLS, bool PL = false>
 __global__ void __launch_bounds__(256, CLS == 1 ? ME_BIG_BLOCKS : ME_MIN_BLOCKS) k_me_chroma(const P* __restrict__ fenc, int fstride, const P* const* __restrict__ refs, int rstride,
                                                            MeChromaArgs ch, const uint16_t* __restrict__ mvcost, const x265cu_me_job* __restrict__ jobs, int n,
                                                            int32_t* __restrict__ out, MeState* __restrict__ state, int* __restrict__ counter,
-                                                           const int32_t* __restrict__ order = nullptr, int order0 = 0)
+                                                           const int32_t* __restrict__ order = nullptr, int order0 = 0, int ppitch = 0)
 {
     extern __shared__ unsigned char me_smem[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -1731,42 +1772,44 @@ __global__ void __launch_bounds__(256, CLS == 1 ? ME_BIG_BLOCKS : ME_MIN_BLOCKS)
         const x265cu_me_job j = jobs[jid];
         MeCtx<P> c;
         me_make_ctx<P>(c, j, fenc, fstride, refs, rstride, 0, mvcost, lane, sm);
+        if (PL) c.ppitch = ppitch;
         if (me_subpel_class(c) != CLS) continue;                   // the sibling launch owns this job
         MeChromaCtx<P> cc;
         me_set_chroma<P>(cc, c, j, ch, fstride);
         MeState st;
-        if (PHASE == 1) { me_phase1<P, CLS, true>(c, j, st, &cc); if (lane == 0) state[jid] = st; }
-        else            { st = state[jid]; me_phase3<P, CLS, true>(c, j, st, out + (size_t)jid * 4, &cc); }
+        if (PHASE == 1) { me_phase1<P, CLS, true, PL>(c, j, st, &cc); if (lane == 0) state[jid] = st; }
+        else            { st = state[jid]; me_phase3<P, CLS, true, PL>(c, j, st, out + (size_t)jid * 4, &cc); }
         __syncwarp();
     }
 }
 
-template <typename P, int PHASE, int CLS>
+template <typename P, int PHASE, int CLS, bool PL = false>
 static int launch_me_chroma_phase(x265cu_ctx* ctx, const void* fenc, int fstride, const void* const* refs, int rstride, const MeChromaArgs& ch,
                                   const uint16_t* mvcost, const x265cu_me_job* jobs, int n, int32_t* out, MeState* state, int* counter,
-                                  const int32_t* order = NULL, int order0 = 0)
+                                  const int32_t* order = NULL, int order0 = 0, int ppitch = 0)
 {
     const int threads = 256, warps = threads / 32;
-    const size_t smem = sizeof(MeShared) * warps;
+    const size_t smem = PL ? 0 : sizeof(MeShared) * warps;            // the phase-plane path never touches the interpolation scratch
     int blocks = ctx->sm_count * (CLS == 1 ? ME_BIG_BLOCKS : ME_MIN_BLOCKS);
     int need = (n + warps - 1) / warps;
     if (blocks > need) blocks = need;
-    k_me_chroma<P, PHASE, CLS><<<blocks, threads, smem, ctx->stream>>>((const P*)fenc, fstride, (const P* const*)refs, rstride, ch, mvcost, jobs, n, out, state, counter, order, order0);
+    k_me_chroma<P, PHASE, CLS, PL><<<blocks, threads, smem, ctx->stream>>>((const P*)fenc, fstride, (const P* const*)refs, rstride, ch, mvcost, jobs, n, out, state, counter, order, order0, ppitch);
     CU_LAUNCH_CHECK(ctx);
     return 0;
 }
 
-template <typename P, int PHASE, int CLS>
+template <typename P, int PHASE, int CLS, bool PL = false>
 static int launch_me_phase(x265cu_ctx* ctx, const void* fenc, int fstride, const void* const* refs, int rstride, int lowres,
                            const uint16_t* mvcost, const x265cu_me_job* jobs, int n, int32_t* out, MeState* state, int* counter,
-                           const int32_t* list = NULL, const int* list_n = NULL, const int32_t* order = NULL, int order0 = 0)
+                           const int32_t* list = NULL, const int* list_n = NULL, const int32_t* order = NULL, int order0 = 0, int ppitch = 0)
 {
     const int threads = 256, warps = threads / 32;
-    const size_t smem = PHASE == 2 ? 0 : sizeof(MeShared) * warps;      // the integer search never touches the interpolation scratch
+    // the integer search and the phase-plane path never touch the interpolation scratch
+    const size_t smem = (PHASE == 2 || PL) ? 0 : sizeof(MeShared) * warps;
     int blocks = ctx->sm_count * (PHASE == 2 ? ME_P2_BLOCKS : (CLS == 1 ? ME_BIG_BLOCKS : ME_MIN_BLOCKS));
     int need = (n + warps - 1) / warps;
     if (blocks > need) blocks = need;
-    k_me<P, PHASE, CLS><<<blocks, threads, smem, ctx->stream>>>((const P*)fenc, fstride, (const P* const*)refs, rstride, lowres, mvcost, jobs, n, out, state, counter, list, list_n, order, order0);
+    k_me<P, PHASE, CLS, PL><<<blocks, threads, smem, ctx->stream>>>((const P*)fenc, fstride, (const P* const*)refs, rstride, lowres, mvcost, jobs, n, out, state, counter, list, list_n, order, order0, ppitch);
     CU_LAUNCH_CHECK(ctx);
     return 0;
 }
@@ -1786,10 +1829,33 @@ template <typename P>
 static int launch_me_window(x265cu_ctx* ctx, const void* fenc, int fstride, const uint16_t* mvcost, const x265cu_me_job* jobs,
                             MeState* st, const MeWinLaunch& w);
 
+// the two PU-class launches (small pow2 PUs, everything else) of a pre-check (PHASE 1) or sub-pel (PHASE 3) pass;
+// `counter_dev` = the first of their two job counters
+template <typename P, int PHASE, bool PL>
+static int launch_me_classes(x265cu_ctx* ctx, const void* fenc, int fstride, const void* const* refs, int rstride, int lowres,
+                             const uint16_t* mvcost, const x265cu_me_job* jobs, int n, int32_t* out, MeState* st, int* counter_dev,
+                             const MeChromaArgs* ch, const int32_t* ord, int ord0, int ppitch)
+{
+    int rc = 0;
+    if (ch)
+    {
+        rc |= launch_me_chroma_phase<P, PHASE, 0, PL>(ctx, fenc, fstride, refs, rstride, *ch, mvcost, jobs, n, out, st, counter_dev + 0, ord, ord0, ppitch);
+        rc |= launch_me_chroma_phase<P, PHASE, 1, PL>(ctx, fenc, fstride, refs, rstride, *ch, mvcost, jobs, n, out, st, counter_dev + 1, ord, ord0, ppitch);
+    }
+    else
+    {
+        rc |= launch_me_phase<P, PHASE, 0, PL>(ctx, fenc, fstride, refs, rstride, lowres, mvcost, jobs, n, out, st, counter_dev + 0, NULL, NULL, ord, ord0, ppitch);
+        rc |= launch_me_phase<P, PHASE, 1, PL>(ctx, fenc, fstride, refs, rstride, lowres, mvcost, jobs, n, out, st, counter_dev + 1, NULL, NULL, ord, ord0, ppitch);
+    }
+    return rc;
+}
+
+// ppitch != 0: the references carry quarter-pel phase planes ppitch bytes apart (frame analyser); the pre-check and
+// sub-pel launches then read their candidates from them
 template <typename P>
 static int launch_me_t(x265cu_ctx* ctx, const void* fenc, int fstride, const void* const* refs, int rstride, int lowres,
                        const uint16_t* mvcost, const x265cu_me_job* jobs, int n, int32_t* out, MeState* st, int* counter_dev,
-                       const MeChromaArgs* ch, const MeWinLaunch* win)
+                       const MeChromaArgs* ch, const MeWinLaunch* win, int ppitch)
 {
     int rc = 0;
     // shape-sorted job order (geometry.h `order`), measured on B200 at 2160p (profiles/me_r2_ncu.md section 5): it helps kernels
@@ -1802,16 +1868,8 @@ static int launch_me_t(x265cu_ctx* ctx, const void* fenc, int fstride, const voi
     const int32_t* ord = ordMode >= 2 ? ordAll : NULL;                       // pre-checks, luma-only sub-pel
     const int32_t* ord3 = (ordMode >= 2 || (ordMode == 1 && ch)) ? ordAll : NULL;   // chroma sub-pel
     const int ord0 = win ? win->job0 : 0;
-    if (ch)
-    {
-        rc |= launch_me_chroma_phase<P, 1, 0>(ctx, fenc, fstride, refs, rstride, *ch, mvcost, jobs, n, out, st, counter_dev + 0, ord, ord0);
-        rc |= launch_me_chroma_phase<P, 1, 1>(ctx, fenc, fstride, refs, rstride, *ch, mvcost, jobs, n, out, st, counter_dev + 1, ord, ord0);
-    }
-    else
-    {
-        rc |= launch_me_phase<P, 1, 0>(ctx, fenc, fstride, refs, rstride, lowres, mvcost, jobs, n, out, st, counter_dev + 0, NULL, NULL, ord, ord0);
-        rc |= launch_me_phase<P, 1, 1>(ctx, fenc, fstride, refs, rstride, lowres, mvcost, jobs, n, out, st, counter_dev + 1, NULL, NULL, ord, ord0);
-    }
+    rc |= ppitch ? launch_me_classes<P, 1, true>(ctx, fenc, fstride, refs, rstride, lowres, mvcost, jobs, n, out, st, counter_dev + 0, ch, ord, ord0, ppitch)
+                 : launch_me_classes<P, 1, false>(ctx, fenc, fstride, refs, rstride, lowres, mvcost, jobs, n, out, st, counter_dev + 0, ch, ord, ord0, 0);
     CU_CHECK(cudaEventRecord(ctx->me_ev[1], ctx->stream));
     if (win && !lowres)
     {
@@ -1822,22 +1880,15 @@ static int launch_me_t(x265cu_ctx* ctx, const void* fenc, int fstride, const voi
     else
         rc |= launch_me_phase<P, 2, -1>(ctx, fenc, fstride, refs, rstride, lowres, mvcost, jobs, n, out, st, counter_dev + 2);
     CU_CHECK(cudaEventRecord(ctx->me_ev[2], ctx->stream));
-    if (ch)
-    {
-        rc |= launch_me_chroma_phase<P, 3, 0>(ctx, fenc, fstride, refs, rstride, *ch, mvcost, jobs, n, out, st, counter_dev + 3, ord3, ord0);
-        rc |= launch_me_chroma_phase<P, 3, 1>(ctx, fenc, fstride, refs, rstride, *ch, mvcost, jobs, n, out, st, counter_dev + 4, ord3, ord0);
-    }
-    else
-    {
-        rc |= launch_me_phase<P, 3, 0>(ctx, fenc, fstride, refs, rstride, lowres, mvcost, jobs, n, out, st, counter_dev + 3, NULL, NULL, ord, ord0);
-        rc |= launch_me_phase<P, 3, 1>(ctx, fenc, fstride, refs, rstride, lowres, mvcost, jobs, n, out, st, counter_dev + 4, NULL, NULL, ord, ord0);
-    }
+    const int32_t* ordS = ch ? ord3 : ord;
+    rc |= ppitch ? launch_me_classes<P, 3, true>(ctx, fenc, fstride, refs, rstride, lowres, mvcost, jobs, n, out, st, counter_dev + 3, ch, ordS, ord0, ppitch)
+                 : launch_me_classes<P, 3, false>(ctx, fenc, fstride, refs, rstride, lowres, mvcost, jobs, n, out, st, counter_dev + 3, ch, ordS, ord0, 0);
     return rc;
 }
 
 static int launch_me(x265cu_ctx* ctx, int depth, const void* fenc, int fstride, const void* const* refs, int rstride, int lowres,
                      const uint16_t* mvcost, const x265cu_me_job* jobs, int n, int32_t* out, int* counter_dev, const MeChromaArgs* chroma = NULL,
-                     const MeWinLaunch* win = NULL)
+                     const MeWinLaunch* win = NULL, int ppitch = 0)
 {
     if (n <= 0) return 0;
     CU_CHECK(cudaMemsetAsync(counter_dev, 0, 8 * sizeof(int), ctx->stream));
@@ -1852,8 +1903,9 @@ static int launch_me(x265cu_ctx* ctx, int depth, const void* fenc, int fstride, 
     MeState* st = (MeState*)ctx->d_me_state;
     CU_CHECK(cudaEventRecord(ctx->me_ev[0], ctx->stream));
     if (chroma && lowres) chroma = NULL;                    // the lowres planes have no chroma (lowres.h)
-    const int rc = depth == 8 ? launch_me_t<uint8_t>(ctx, fenc, fstride, refs, rstride, lowres, mvcost, jobs, n, out, st, counter_dev, chroma, win)
-                              : launch_me_t<uint16_t>(ctx, fenc, fstride, refs, rstride, lowres, mvcost, jobs, n, out, st, counter_dev, chroma, win);
+    if (lowres) ppitch = 0;
+    const int rc = depth == 8 ? launch_me_t<uint8_t>(ctx, fenc, fstride, refs, rstride, lowres, mvcost, jobs, n, out, st, counter_dev, chroma, win, ppitch)
+                              : launch_me_t<uint16_t>(ctx, fenc, fstride, refs, rstride, lowres, mvcost, jobs, n, out, st, counter_dev, chroma, win, ppitch);
     CU_CHECK(cudaEventRecord(ctx->me_ev[3], ctx->stream));
     return rc;
 }

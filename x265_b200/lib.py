@@ -287,6 +287,9 @@ _AN_PROTOS = {
     "x265cu_analyser_enable_chroma": (I, [P]),
     "x265cu_analyser_set_ref_chroma": (I, [P, I, P, P, I]),
     "x265cu_analyser_load_chroma": (I, [P, P, P, I]),
+    "x265cu_analyser_phase_planes_ms": (I, [P, C.POINTER(C.c_float)]),
+    "x265cu_analyser_ref_plane_phase": (P, [P, I, I]),
+    "x265cu_analyser_phase_region": (I, [P, I, C.POINTER(I)]),
 }
 _AN_PROTOS["x265cu_propagate_cost_batch"] = (I, [P, P, P, P, P, P, C.c_double, I64])
 _AN_PROTOS["x265cu_lowres_intra_batch"] = (I, [P, I, P, I, I, I, I, I])
@@ -410,6 +413,31 @@ class Analyser:
 
     def ref_updated(self, idx):
         self.lib.check(self.lib.L.x265cu_analyser_ref_updated(self.h, idx))
+
+    # ---- quarter-pel phase planes of the references (X265CU_ME_PHASEPLANES) ----
+    def phase_planes_ms(self):
+        """Device ms of the last run's phase-plane build (0.0 when it built none)."""
+        ms = C.c_float()
+        self.lib.check(self.lib.L.x265cu_analyser_phase_planes_ms(self.h, C.byref(ms)))
+        return float(ms.value)
+
+    def phase_region(self, idx):
+        """(x0, x1, y0, y1): the picture rectangle of reference idx's phase planes that the last run built."""
+        box = (I * 4)()
+        self.lib.check(self.lib.L.x265cu_analyser_phase_region(self.h, idx, box))
+        return tuple(int(v) for v in box)
+
+    def fetch_phase_plane(self, idx, phase):
+        """Phase plane (yFrac << 2) | xFrac of reference idx, margins included: (height + 160) x stride, pixel (0, 0) at
+        row 80, column 96."""
+        ptr = self.lib.L.x265cu_analyser_ref_plane_phase(self.h, idx, phase)
+        if not ptr:
+            raise RuntimeError("no phase plane %d of reference %d" % (phase, idx))
+        es = np.dtype(self.dtype).itemsize
+        out = np.zeros((self.height + 160, self.stride), self.dtype)
+        self.lib.check(self.lib.L.x265cu_d2h(self.lib.ctx, out.ctypes.data, ptr - (80 * self.stride + 96) * es, out.nbytes))
+        self.lib.sync()
+        return out
 
     def fetch(self, what):
         es = np.dtype(self.dtype).itemsize
